@@ -2,6 +2,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-secondary] [--no-cpu-baseline]
                     [--workload hifigan_cfg2|fregan_cfg2|wavernn_cfg1|wavernn_cfg3|tacotron_cfg4|e2e_cfg5] [--precision ...]
+                    [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  The headline is BASELINE.json configs[1] (the config the metric is quoted on): HiFi-GAN
 Generator forward, batch 32 random mels of 256 frames x 80 bins per GPU; a "step" is one forward over one batch; under
@@ -20,6 +21,9 @@ torchrun every rank runs its own batch (weak scaling: utterance batches shard ac
              tacotron_cfg4 (configs[3]), e2e_cfg5 (configs[4], weak: 128 utterances per GPU; strong: 1024 utterances
              over N GPUs), hifigan_fp32_equivalent (3-term split everywhere), and at N > 1 the fold-sharded cfg 3
 --impl reference: the CPU implementation (oracle port, all host threads) on the same config (rank 0 only).
+--dump-outputs DIR: after the timed steps, rank 0 writes the waveforms its last timed step returned (the whole batch,
+             float32 [32, 1, 51200], 6.6 MB) to DIR/wav.npy.  Inputs and weights are seeded, so two builds run with the same
+             arguments can be compared output for output (GAN workloads: hifigan_cfg2, fregan_cfg2).
 """
 from __future__ import annotations
 
@@ -50,8 +54,15 @@ def parse():
     ap.add_argument("--soak-seconds", type=float, default=2.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="headline workload only")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the waveforms of the last timed step to DIR/wav.npy (hifigan_cfg2 / fregan_cfg2)")
     ap.add_argument("--cpu-child", nargs=3, default=None, help=argparse.SUPPRESS)
-    return ap.parse_args()
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs is not None and (args.impl != "ours" or args.workload not in ("hifigan_cfg2", "fregan_cfg2")):
+        ap.error("--dump-outputs needs --impl ours and --workload hifigan_cfg2 or fregan_cfg2")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -130,8 +141,9 @@ def run_reference(args):
 # ------------------------------------------------------------------------------------------------
 # ------------------------------------------------------------------------------------------------
 def measure_hifigan(ctx: Ctx, args, workload: str, precision: str, steps: int, warmup: int, soak_s: float, cpu: bool,
-                    roofline: bool = True):
-    """HiFi-GAN / Fre-GAN generator forward on the cfg-2 batch shape; returns the JSON dict (rank 0) or None."""
+                    roofline: bool = True, dump_dir: str | None = None):
+    """HiFi-GAN / Fre-GAN generator forward on the cfg-2 batch shape; returns the JSON dict (rank 0) or None.
+    dump_dir: rank 0 writes the waveforms of the last timed resident step there as wav.npy."""
     import numpy as np
     import torch
 
@@ -159,9 +171,10 @@ def measure_hifigan(ctx: Ctx, args, workload: str, precision: str, steps: int, w
     samples_per_step = B * T * hop
     lib = _lib.lib()
     produced = {"n": 0}
+    last = {}
 
     def step_resident():
-        g(mel_dev)
+        last["wav"] = g(mel_dev)
 
     def step_e2e():
         wavs = mod.infer_waveforms(mels_np, batch_size=B)   # host numpy in, host numpy out, host sync inside
@@ -172,6 +185,11 @@ def measure_hifigan(ctx: Ctx, args, workload: str, precision: str, steps: int, w
     r = ctx.timed(step_resident, steps, max(3, warmup), soak_s)
     launches_total = int(lib.mb_launch_count() - l0)
     launches = int(round(launches_total * steps / (max(3, warmup) + 2 * steps + r["soak_steps"])))
+    if dump_dir is not None and rank == 0:
+        out = Path(dump_dir)
+        out.mkdir(parents=True, exist_ok=True)
+        np.save(out / "wav.npy", last["wav"].float().cpu().numpy())
+        log(f"dumped {out / 'wav.npy'}")
     log(f"resident: soaked {r['ms'] / steps:.3f} ms/step, burst {r['ms_burst'] / steps:.3f}; e2e pass")
     e = ctx.timed(step_e2e, steps, 2, min(soak_s, 1.0), host_clock=True)
     assert produced["n"] == samples_per_step
@@ -281,7 +299,8 @@ def run_ours(args):
     try:
         cpu = (not args.no_cpu_baseline) and ctx.world == 1
         if args.workload in ("hifigan_cfg2", "fregan_cfg2"):
-            line = measure_hifigan(ctx, args, args.workload, args.precision, args.steps, args.warmup, args.soak_seconds, cpu)
+            line = measure_hifigan(ctx, args, args.workload, args.precision, args.steps, args.warmup, args.soak_seconds, cpu,
+                                   dump_dir=args.dump_outputs)
             secondary = {}
             if args.workload == "hifigan_cfg2" and not args.no_secondary:
                 import bench_e2e
@@ -319,10 +338,10 @@ def run_ours(args):
             import bench_tacotron
             import bench_wavernn
 
-            fn = {"wavernn_cfg1": lambda: bench_wavernn.measure_cfg1(ctx, args, cpu),
-                  "wavernn_cfg3": lambda: bench_wavernn.measure_cfg3(ctx, args, cpu, steps=max(3, min(args.steps, 5))),
-                  "tacotron_cfg4": lambda: bench_tacotron.measure(ctx, args, cpu, steps=max(1, min(args.steps, 10))),
-                  "e2e_cfg5": lambda: bench_e2e.measure(ctx, args, cpu, steps=max(1, min(args.steps, 5)))}[args.workload]
+            fn = {"wavernn_cfg1": lambda: bench_wavernn.measure_cfg1(ctx, args, cpu, steps=args.steps),
+                  "wavernn_cfg3": lambda: bench_wavernn.measure_cfg3(ctx, args, cpu, steps=args.steps),
+                  "tacotron_cfg4": lambda: bench_tacotron.measure(ctx, args, cpu, steps=args.steps),
+                  "e2e_cfg5": lambda: bench_e2e.measure(ctx, args, cpu, steps=args.steps)}[args.workload]
             line = fn()
             if ctx.rank == 0:
                 print(json.dumps(line), flush=True)

@@ -3,14 +3,17 @@
 gcc -O2 -ffp-contract=off so that every a*b+c stays two rounded operations unless written as
 fmaf() - the arithmetic contract shared with the CUDA kernel (include/mb_wavernn_math.h).
 The reference is pure Python with ONE compiled piece on the edge of the path: monotonic_align/core.pyx (Cython, 42 lines;
-SURVEY.md 8f row N4).  build_ref() compiles THAT FILE, from where it lies under /root/reference, with `cython` + gcc into
-oracle/_ref/monotonic_align_core*.so (git-ignored, travels to the GPU box) - the real reference for that row; nothing of the
-reference is copied into the repo.  Everything else has no C/C++ reference to compile.
+SURVEY.md 8f row N4).  build_ref() compiles THAT FILE, from where it lies in the reference tree (ref_harness.REFERENCE_ROOT),
+with `cython` + gcc into oracle/_ref/monotonic_align_core*.so (git-ignored) - the real reference for that row, whose outputs
+oracle/make_golden_pinned.py stores for the tests; nothing of the reference is copied into the repo.  Everything else has no
+C/C++ reference to compile.
 """
 from __future__ import annotations
 
 import subprocess
 from pathlib import Path
+
+from ref_harness import REFERENCE_ROOT
 
 HERE = Path(__file__).resolve().parent
 SRC = HERE / "wavernn_twin.c"
@@ -28,7 +31,7 @@ def build(force: bool = False) -> Path:
 
 
 REF_DIR = HERE / "_ref"
-REF_PYX = Path("/root/reference/monotonic_align/core.pyx")
+REF_PYX = REFERENCE_ROOT / "monotonic_align" / "core.pyx"
 
 
 def ref_so():
@@ -38,7 +41,7 @@ def ref_so():
 
 
 def build_ref(force: bool = False):
-    """compile the reference's own monotonic_align/core.pyx into oracle/_ref (container only: needs /root/reference)"""
+    """compile the reference's own monotonic_align/core.pyx into oracle/_ref (needs the reference tree)"""
     import sysconfig
 
     if not REF_PYX.is_file():

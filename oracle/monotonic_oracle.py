@@ -4,7 +4,9 @@
                        monotonic_align/__init__.py:6-19 (float32 DP in place, int32 path)
   reference_core()     the reference's OWN core.pyx compiled by oracle/build_oracle.build_ref() into oracle/_ref (the module's
                        init symbol is PyInit_core, so it is loaded under the name "core")
-tests/test_monotonic.py checks restatement == compiled reference (bit-identical values and paths) and CUDA == both."""
+  random_case()        the seeded inputs of tests/test_monotonic.py
+oracle/make_golden_pinned.py stores the compiled reference's paths and values on those inputs; tests/test_monotonic.py checks
+restatement == compiled reference (bit-identical values and paths) and CUDA == both."""
 from __future__ import annotations
 
 import importlib.machinery
@@ -51,3 +53,13 @@ def maximum_path_numpy(neg_cent: np.ndarray, t_ys: np.ndarray, t_xs: np.ndarray)
     for b in range(values.shape[0]):
         maximum_path_each(paths[b], values[b], int(t_ys[b]), int(t_xs[b]))
     return paths, values
+
+
+def random_case(seed: int, b: int, ty: int, tx: int):
+    """-> (neg_cent float32 [b, ty, tx], t_ys int32 [b], t_xs int32 [b]); row 0 spans the whole grid"""
+    rng = np.random.RandomState(seed)
+    v = (rng.randn(b, ty, tx) * 3).astype(np.float32)
+    t_ys = rng.randint(max(1, ty // 2), ty + 1, size=b).astype(np.int32)
+    t_xs = np.minimum(rng.randint(1, tx + 1, size=b), t_ys).astype(np.int32)  # a monotonic path needs t_x <= t_y
+    t_ys[0], t_xs[0] = ty, min(tx, ty)
+    return v, t_ys, t_xs

@@ -1,6 +1,7 @@
 """CPU tests: the C-ABI library loads and exports every symbol include/mockingbird_b200.h declares;
 handle creation / plan building / error paths work without a GPU (no compute calls)."""
 import ctypes as C
+import json
 import re
 from pathlib import Path
 
@@ -108,23 +109,17 @@ def test_generator_without_cuda_fails_loudly():
         g.to("cpu")
 
 
-def test_text_front_end_matches_reference_ids():
-    """symbols table (utils/symbols.py:18) and basic_cleaners text_to_sequence (utils/text.py:13-40)"""
+def test_text_front_end_matches_reference_ids(golden_dir):
+    """symbols table (utils/symbols.py:18) and basic_cleaners text_to_sequence (utils/text.py:13-40); the reference's ids
+    are stored by oracle/make_golden_pinned.py"""
     from mockingbird_b200.synthesizer.utils.symbols import symbols
     from mockingbird_b200.synthesizer.utils.text import text_to_sequence
 
     assert len(symbols) == 75 and symbols[0] == "_" and symbols[1] == "~"
     assert text_to_sequence("Hello  World 1", ["basic_cleaners"]) == [35, 32, 39, 39, 42, 74, 50, 42, 45, 39, 31, 74, 54, 1]
-    try:
-        import ref_harness as rh
-    except ImportError:
-        return
-    if rh.reference_available():
-        rh.install()
-        from models.synthesizer.utils.text import text_to_sequence as ref_tts
-
-        for t in ["ni3 hao3 shi4 jie4", "Mixed CASE,  spaces!", "~_skip~"]:
-            assert text_to_sequence(t, ["basic_cleaners"]) == ref_tts(t, ["basic_cleaners"])
+    pinned = json.loads((golden_dir / "reference_pinned.json").read_text())
+    for case in pinned["text_to_sequence"]:
+        assert text_to_sequence(case["text"], ["basic_cleaners"]) == case["ids"], case["text"]
 
 
 def test_tacotron_handle_and_missing_weight_errors():

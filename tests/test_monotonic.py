@@ -1,53 +1,47 @@
-"""monotonic_align.maximum_path (SURVEY.md 8f row N4): numpy restatement == the reference's own compiled core.pyx (oracle/_ref,
-built by oracle/build_oracle.build_ref() in the build container; travels to the GPU box) == the CUDA wavefront DP."""
+"""monotonic_align.maximum_path (SURVEY.md 8f row N4): numpy restatement == the reference's own compiled core.pyx == the CUDA
+wavefront DP.  The compiled reference's paths and DP values on these cases are stored by oracle/make_golden_pinned.py."""
+import json
+
 import numpy as np
 import pytest
 import torch
 
+import make_golden_pinned as mgp
 import monotonic_oracle as mo
 
 
-def _case(seed, b, ty, tx):
-    rng = np.random.RandomState(seed)
-    v = (rng.randn(b, ty, tx) * 3).astype(np.float32)
-    t_ys = rng.randint(max(1, ty // 2), ty + 1, size=b).astype(np.int32)
-    t_xs = np.minimum(rng.randint(1, tx + 1, size=b), t_ys).astype(np.int32)  # a monotonic path needs t_x <= t_y
-    t_ys[0], t_xs[0] = ty, min(tx, ty)
-    return v, t_ys, t_xs
+@pytest.fixture(scope="module")
+def golden(golden_dir):
+    return json.loads((golden_dir / "reference_pinned.json").read_text()), np.load(golden_dir / "reference_pinned.npz")
 
 
-@pytest.mark.parametrize("shape", [(3, 37, 11), (2, 1, 1), (4, 64, 64), (2, 300, 75)])
-def test_restatement_equals_compiled_reference(shape):
-    core = mo.reference_core()
-    if core is None:
-        pytest.skip("oracle/_ref not built (needs /root/reference once)")
-    v, t_ys, t_xs = _case(1, *shape)
-    p_ref, v_ref = np.zeros(v.shape, np.int32), v.copy()
-    core.maximum_path_c(p_ref, v_ref, t_ys, t_xs)
+def _reference_path(golden, seed, shape):
+    bits = golden[1][mgp.monotonic_key(seed, shape) + "_path"]
+    return np.unpackbits(bits, count=int(np.prod(shape))).reshape(shape).astype(np.int32)
+
+
+@pytest.mark.parametrize("shape", mgp.MONOTONIC_CASES[1])
+def test_restatement_equals_compiled_reference(shape, golden):
+    v, t_ys, t_xs = mo.random_case(1, *shape)
     p, vv = mo.maximum_path_numpy(v, t_ys, t_xs)
-    assert np.array_equal(p, p_ref) and np.array_equal(vv, v_ref)
+    assert np.array_equal(p, _reference_path(golden, 1, shape))
+    assert mgp.array_digest(vv) == golden[0]["monotonic_values"][mgp.monotonic_key(1, shape)]
     assert np.array_equal(p.sum(axis=(1, 2)), t_ys)  # one cell per frame
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("shape", [(3, 37, 11), (2, 1, 1), (4, 64, 64), (16, 1000, 200), (2, 300, 75)])
-def test_cuda_equals_reference(shape):
+@pytest.mark.parametrize("shape", mgp.MONOTONIC_CASES[2])
+def test_cuda_equals_reference(shape, golden):
     from mockingbird_b200.monotonic_align import maximum_path
 
-    v, t_ys, t_xs = _case(2, *shape)
+    v, t_ys, t_xs = mo.random_case(2, *shape)
     b, ty, tx = shape
     mask = np.zeros((b, ty, tx), np.float32)
     for i in range(b):
         mask[i, : t_ys[i], : t_xs[i]] = 1
     got = maximum_path(torch.from_numpy(v).cuda(), torch.from_numpy(mask).cuda())
     assert got.dtype == torch.float32 and got.shape == (b, ty, tx)
-    core = mo.reference_core()
-    if core is not None:
-        p_ref, v_ref = np.zeros(v.shape, np.int32), v.copy()
-        core.maximum_path_c(p_ref, v_ref, t_ys, t_xs)
-    else:
-        p_ref, _ = mo.maximum_path_numpy(v, t_ys, t_xs)
-    assert np.array_equal(got.cpu().numpy().astype(np.int32), p_ref)
+    assert np.array_equal(got.cpu().numpy().astype(np.int32), _reference_path(golden, 2, shape))
     # size-independent properties: exactly one cell per valid frame, monotone non-decreasing column, ends at the corners
     g = got.cpu().numpy()
     for i in range(b):

@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 import torch
 
-import ref_harness as rh
+import make_golden_pinned as mgp
 import ref_init as ri
 import wavernn_oracle as wo
 
@@ -80,16 +80,12 @@ def test_builtin_noise_is_exp1():
     assert q.min() > 0 and abs(q.mean() - 1.0) < 0.03 and abs(q.var() - 1.0) < 0.08
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not rh.reference_available(), reason="/root/reference not present")
-def test_ref_init_wavernn_bit_identical_to_reference_constructor():
-    rh.install()
-    rh.hide_cuda()
-    m = rh.build_wavernn(seed=4)
+def test_ref_init_wavernn_bit_identical_to_reference_constructor(golden_dir):
+    """names, dtypes, shapes and bits of the state dict == the reference constructor's (digest stored by
+    oracle/make_golden_pinned.py)"""
+    pinned = json.loads((golden_dir / "reference_pinned.json").read_text())
     sd = ri.wavernn_state_dict(4, randomize_bn=False)
-    ref = m.state_dict()
-    assert set(sd) == set(ref)
-    assert all(torch.equal(sd[k], ref[k]) for k in sd)
+    assert mgp.state_dict_digest(sd) == pinned["state_dicts"]["wavernn_seed4"]
 
 
 def test_three_term_fp16_split_is_fp32_equivalent():
